@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of proxtv_b200:  tv1_2d (DR2_TV) Mpixels/s on 4096 x 4096 float64 images, lambda = 0.2.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--size M] [--engine auto|lane|lane-t|chunked|seq]
-                    [--workload cfg2|cfg3|cfg4|cfg5|split] [--batch B] [--pieces P]
+                    [--workload cfg2|cfg3|cfg4|cfg5|split] [--batch B] [--pieces P] [--dump-outputs DIR]
 
 One "step" = one complete solve (35 Douglas-Rachford iterations + the final projection pair, 72 fiber passes) of one
 4096 x 4096 image per GPU (BASELINE.json configs[1]; synthetic piecewise-constant + Gaussian-noise input, SURVEY.md 8d).
@@ -19,6 +19,9 @@ Rank 0 prints ONE JSON line.  Keys beyond the base contract:
 --impl reference times only that CPU implementation (rank 0 alone), same metric/config.
 --workload cfg3 | cfg4 | cfg5: the other BASELINE.json configurations (cfg5 over N GPUs: NCCL scatter / gather of image slabs,
 pipelined); --workload split: ONE image over all N ranks (strong scaling; two all-to-alls per iteration).
+--dump-outputs DIR (cfg2): after the timed steps, rank 0 writes what its last timed step returned, DIR/x.npy (the solved image, or
+                a fixed seeded sample of its rows when it is larger than 32 MiB) and DIR/info.npy (DR2_TV's info[]), float64.  The
+                inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -35,6 +38,17 @@ sys.path.insert(0, ROOT)
 
 B_PER_PIXEL_SOLVE = lambda b, maxit=35: b * (1 + 6 * maxit + 5)      # noqa: E731  SURVEY.md 8d: M*N*b*(1 + 6*maxit + 5)
 LAM = 0.2
+DUMP_BYTES = 32 << 20
+
+
+def dump_outputs(d, image, info):
+    """--dump-outputs: the image whole if it fits DUMP_BYTES, else the rows of a fixed seeded sample (sorted), float64."""
+    M, N = image.shape
+    if image.nbytes > DUMP_BYTES:
+        image = image[np.sort(np.random.default_rng(0).choice(M, DUMP_BYTES // (8 * N), replace=False))]
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "x.npy"), np.ascontiguousarray(image, dtype=np.float64))
+    np.save(os.path.join(d, "info.npy"), np.asarray(info, dtype=np.float64))
 
 
 def ncu_traffic(cls=-1, lane_t=False):
@@ -308,7 +322,12 @@ def main():
     ap.add_argument("--workload", default="cfg2", choices=["cfg2", "cfg3", "cfg4", "cfg5", "split"])
     ap.add_argument("--batch", type=int, default=0, help="cfg3: signals; cfg5: images per GPU (0 = BASELINE.json's)")
     ap.add_argument("--pieces", type=int, default=4, help="cfg5: pipelined transfer pieces per GPU slab")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="cfg2: write the last timed step's result to DIR (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps: at least one timed step")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "cfg2"):
+        ap.error("--dump-outputs: the cfg2 workload of --impl ours only")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
@@ -360,6 +379,8 @@ def main():
     e1.record(st)
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out.cpu().numpy().T, info)        # out holds the column-major image
     kms = (C.c_double * 3)(); kl = (C.c_longlong * 3)(); ks = (C.c_longlong * 3)()
     lib.proxtv_profile_read(kms, kl, ks)
     launches_timed_region = int(sum(kl[i] for i in range(3)))

@@ -15,7 +15,23 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
-    return np.load(os.path.join(ROOT, "tests", "golden", "golden_v1.npz"))
+    """golden_v1.npz as a dict.  Inputs made by synth_inputs are stored as their call ("<name>_cfg2": M, N, seed, block;
+    "<name>_cfg4": shape..., seed, block) and a digest: they are regenerated here and must match the digest."""
+    from oracle import oracle as O
+    g = dict(np.load(os.path.join(ROOT, "tests", "golden", "golden_v1.npz")))
+    for key in [k for k in g if k.endswith(("_cfg2", "_cfg4"))]:
+        name, p = key[:-5], [int(v) for v in g.pop(key)]
+        x = O.gen_cfg2(p[0], p[1], seed=p[2], block=p[3]) if key.endswith("_cfg2") else O.gen_cfg4(tuple(p[:-2]), seed=p[-2], block=p[-1])
+        assert digest(x) == g.pop(name + "_digest"), "generated input %s differs from the one the reference solved" % name
+        g[name] = x
+    return g
+
+
+@pytest.fixture(scope="session")
+def refcheck():
+    """What the unmodified reference computed on the tests' seeded inputs (tests/golden/make_golden.py reference_checks):
+    digests where a test demands bit-identical results, values (sampled at full size) where it allows a tolerance."""
+    return np.load(os.path.join(ROOT, "tests", "golden", "reference_checks.npz"))
 
 
 @pytest.fixture(scope="session")
@@ -24,14 +40,14 @@ def port():
     return O.Port()
 
 
-@pytest.fixture(scope="session")
-def ref():
-    """The compiled reference, when its prebuilt .so travelled here or /root/reference exists; else skip."""
-    from oracle import oracle as O
-    try:
-        return O.Ref()
-    except Exception as e:  # noqa: BLE001
-        pytest.skip("compiled reference unavailable: %s" % e)
+def digest(a):
+    """64-bit digest of an array's shape and values (float64, or bits for a boolean array): equal digests <=> identical arrays
+    (up to a 2^-64 collision)."""
+    import hashlib
+    a = np.asarray(a)
+    data = np.packbits(a).tobytes() if a.dtype == bool else np.ascontiguousarray(a, dtype="<f8").tobytes()
+    h = hashlib.blake2b(np.asarray(a.shape, dtype="<i8").tobytes() + data, digest_size=8)
+    return np.frombuffer(h.digest(), dtype="<u8")[0]
 
 
 @pytest.fixture(scope="session")

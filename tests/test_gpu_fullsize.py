@@ -1,48 +1,48 @@
-"""GPU parity tests at the BASELINE.json configuration sizes (-m gpu), against the compiled reference (oracle/_ref: the .so is
-built from the unmodified sources by oracle/build_ref.sh and travels to the GPU box; nothing here reads /root/reference) or,
-where the reference has no float32 path, against its float64 result on the float32-rounded input.
+"""GPU parity tests at the BASELINE.json configuration sizes (-m gpu), against what the compiled reference computed on the same
+seeded inputs (tests/golden/reference_checks.npz, made by tests/golden/make_golden.py) or, where the reference has no float32
+path, against its float64 result on the float32-rounded input.  The reference's results are too large to store whole: values are
+compared on seeded samples (whole rows of the 2D results, voxels of the volume) against the max norm of the whole result.
 
 Bars:
   cfg 2  tv1_2d 4096 x 4096 f64         <= 1e-6 relative (max norm; observed ~1e-13) AND identical jump sets on EVERY row and
                                         EVERY column of the result (jump = |x[i+1] - x[i]| > 1e-9, the thresholded form of the
-                                        "break-point index arrays" the reference never returns, SURVEY.md 8c)
+                                        "break-point index arrays" the reference never returns, SURVEY.md 8c): the whole
+                                        boolean jump maps are compared through digests, with per-row / per-column jump counts
+                                        to show where they differ
   cfg 3  tv1w_1d 2048 x 4096 f64        every row bit-exact against the port of tautString_TV1_Weighted
   cfg 4  tvgen 512 x 512 x 256 f32      vs the f64 reference on the f32-rounded input: iteration count equal, stop value within
                                         1e-4 relative, values <= 5e-5 relative (float32 storage of a 35-iteration non-expansive
                                         loop, SURVEY.md 7.3 H5)
   cfg 5  tv1_2d 3 x 2048 x 2048 f32     same float32 bar (<= 5e-5) per image
 """
-import os
-
 import numpy as np
 import pytest
 
-from conftest import jumps, relerr
+from conftest import digest, relerr
 from oracle import oracle as O
 
 pytestmark = pytest.mark.gpu
 
 
-def _threads():
-    try:
-        return max(1, len(os.sched_getaffinity(0)))
-    except AttributeError:
-        return os.cpu_count() or 1
+def jump_maps(x, thr=1e-9):
+    """Boolean jump maps of a 2D result along rows and along columns."""
+    return np.abs(np.diff(x, axis=1)) > thr, np.abs(np.diff(x, axis=0)) > thr
 
 
-def test_cfg2_full_4096_vs_reference_with_jump_sets(ptv, ref):
+def test_cfg2_full_4096_vs_reference_with_jump_sets(ptv, refcheck):
     Y = O.gen_cfg2(4096, 4096, seed=0)
-    want, winfo = ref.dr2_tv(Y, 0.2, n_threads=min(_threads(), 64))
+    assert digest(Y) == refcheck["cfg2_Y"]                 # the seeded input the reference solved
     got = ptv.tv1_2d(Y, 0.2)
-    assert relerr(got, want) <= 1e-6
-    assert relerr(got, want) <= 1e-9                       # what is actually observed: ~1e-13
-    # jump sets of every final-pass fiber (rows) and of every column, vectorised: the boolean jump maps must be identical
-    thr = 1e-9
-    jr_g = np.abs(np.diff(got, axis=1)) > thr; jr_w = np.abs(np.diff(want, axis=1)) > thr
-    jc_g = np.abs(np.diff(got, axis=0)) > thr; jc_w = np.abs(np.diff(want, axis=0)) > thr
-    assert np.array_equal(jr_g, jr_w), "row jump sets differ in %d places" % int((jr_g != jr_w).sum())
-    assert np.array_equal(jc_g, jc_w), "column jump sets differ in %d places" % int((jc_g != jc_w).sum())
-    assert jr_w.sum() > 4_000_000                          # the check is not vacuous: millions of jumps
+    err = np.abs(got[refcheck["cfg2_rows"]] - refcheck["cfg2_want_rows"]).max() / refcheck["cfg2_absmax"]
+    assert err <= 1e-6
+    assert err <= 1e-9                                     # what is actually observed: ~1e-13
+    # jump sets of every final-pass fiber (rows) and of every column: the boolean jump maps must be identical
+    jr_g, jc_g = jump_maps(got)
+    rows = np.nonzero(jr_g.sum(axis=1) != refcheck["cfg2_row_jumps"])[0]
+    cols = np.nonzero(jc_g.sum(axis=0) != refcheck["cfg2_col_jumps"])[0]
+    assert digest(jr_g) == refcheck["cfg2_row_jump_map"], "row jump sets differ; jump counts differ in rows %s" % rows[:20]
+    assert digest(jc_g) == refcheck["cfg2_col_jump_map"], "column jump sets differ; jump counts differ in columns %s" % cols[:20]
+    assert refcheck["cfg2_row_jumps"].sum() > 4_000_000    # the check is not vacuous: millions of jumps
 
 
 def test_cfg3_all_rows_bit_exact(ptv, port):
@@ -52,25 +52,27 @@ def test_cfg3_all_rows_bit_exact(ptv, port):
         assert np.array_equal(G[b], port.tv1_weighted(X[b], W[b])), b
 
 
-def test_cfg4_full_volume_f32(ptv, ref):
+def test_cfg4_full_volume_f32(ptv, refcheck):
     V = O.gen_cfg4((512, 512, 256), seed=0)
     V32 = np.asfortranarray(V.astype(np.float32))
-    want, winfo = ref.pd_tv(np.asfortranarray(V32.astype(np.float64)), [0.2, 0.2, 0.2], [1, 2, 3], n_threads=min(_threads(), 64))
+    assert digest(V32) == refcheck["cfg4_V32"]
+    winfo = refcheck["cfg4_info"]
     got = ptv.tvgen(V32, [0.2, 0.2, 0.2], [1, 2, 3], [1, 1, 1])
     info = ptv.tvgen.last_info
     assert got.dtype == np.float32 and got.shape == V32.shape
     assert info[0] == winfo[0], (info, winfo)              # iterations (35 here: the cap)
     assert abs(info[1] - winfo[1]) <= 1e-4 * abs(winfo[1])
-    assert relerr(got, want) <= 5e-5
+    assert np.abs(got.ravel("F")[refcheck["cfg4_index"]] - refcheck["cfg4_want"]).max() / refcheck["cfg4_absmax"] <= 5e-5
 
 
-def test_cfg5_images_2048_f32(ptv, ref):
+def test_cfg5_images_2048_f32(ptv, refcheck):
     imgs = np.stack([np.ascontiguousarray(O.gen_cfg2(2048, 2048, seed=s)).astype(np.float32) for s in range(3)])
+    assert digest(imgs) == refcheck["cfg5_imgs"]
     got = ptv.tv1_2d_batched(imgs, 0.2)
     assert got.dtype == np.float32 and got.shape == imgs.shape
+    rows = refcheck["cfg5_rows"]
     for s in range(3):
-        want = ref.dr2_tv(np.asfortranarray(imgs[s].astype(np.float64)), 0.2, n_threads=min(_threads(), 64))[0]
-        assert relerr(got[s], want) <= 5e-5, s
+        assert np.abs(got[s][rows] - refcheck["cfg5_want_rows"][s]).max() / refcheck["cfg5_absmax"][s] <= 5e-5, s
 
 
 def test_cfg5_torch_row_major_equals_numpy_path(ptv):
