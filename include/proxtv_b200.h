@@ -114,7 +114,10 @@ int proxtv_set_engine(int engine);
 /* Batched 1D prox over the fibers of a column-major array: nf fibers of len samples, fiber j starting at
  * (j / inc) * inc * len + (j % inc) with element stride inc (the reference's slicing rule, src/TVNDopt.cpp:184-188;
  * inc == 1: nf contiguous signals back to back).  lamv == NULL: uniform weight lam, else per-edge weights laid out the
- * same way with len-1 samples per fiber (batched tautString_TV1_Weighted). */
+ * same way with len-1 samples per fiber (batched tautString_TV1_Weighted).  Unweighted calls with at least 1024 fibers of at least
+ * 64 samples whose shape suits TMA tiling run on the lane engine under engines 0 (auto, while the data passes its guard), 7 and 8:
+ * the result is then the slope-form scan, within ~4e-15 of the reference's linearized taut string but not bit-identical to it.
+ * Engine 2 (chunked) keeps these calls bit-identical to the reference. */
 int proxtv_prox_fibers_dev_f64(const double *in, double *out, long long nf, int len, long long inc, double lam,
                                const double *lamv, void *stream);
 int proxtv_prox_fibers_dev_f32(const float *in, float *out, long long nf, int len, long long inc, float lam,
@@ -191,6 +194,8 @@ int proxtv_lane_prox_dev_f32(int op, const float *A, const float *B, const float
 /* same with a second result array (the ops that write two results: 3 = first half of a Douglas-Rachford iteration, transposed) */
 int proxtv_lane_prox2_dev_f64(int op, const double *A, const double *B, const double *C, double *X, double *X2, long long nf, int len,
                               long long inc, double lam, void *stream);
+int proxtv_lane_prox2_dev_f32(int op, const float *A, const float *B, const float *C, float *X, float *X2, long long nf, int len,
+                              long long inc, float lam, void *stream);
 void proxtv_lane_tuning(int clen, int halo, int variant);
 unsigned long long proxtv_lane_stats(int reset);
 /* Under engine 0 (auto) the solvers use the lane engine only while the data keeps segments short -- penalty not larger than about the

@@ -61,6 +61,7 @@ SIGNATURES = {
     "proxtv_lane_prox_dev_f64": (C.c_int, [C.c_int, _vp, _vp, _vp, _vp, C.c_longlong, C.c_int, C.c_longlong, C.c_double, _vp]),
     "proxtv_lane_prox_dev_f32": (C.c_int, [C.c_int, _vp, _vp, _vp, _vp, C.c_longlong, C.c_int, C.c_longlong, C.c_float, _vp]),
     "proxtv_lane_prox2_dev_f64": (C.c_int, [C.c_int, _vp, _vp, _vp, _vp, _vp, C.c_longlong, C.c_int, C.c_longlong, C.c_double, _vp]),
+    "proxtv_lane_prox2_dev_f32": (C.c_int, [C.c_int, _vp, _vp, _vp, _vp, _vp, C.c_longlong, C.c_int, C.c_longlong, C.c_float, _vp]),
     "proxtv_lane_tuning": (None, [C.c_int, C.c_int, C.c_int]),
     "proxtv_lane_stats": (C.c_ulonglong, [C.c_int]),
     "proxtv_lane_guard_last": (C.c_int, []),

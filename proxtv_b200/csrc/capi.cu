@@ -244,6 +244,15 @@ int proxtv_lane_prox_dev_f32(int op, const float* A, const float* B, const float
     if (e != cudaSuccess) { cudaGetLastError(); g_err = std::string("proxtv_lane_prox_dev_f32: ") + cudaGetErrorString(e); return 0; }
     return 1;
 }
+int proxtv_lane_prox2_dev_f32(int op, const float* A, const float* B, const float* C, float* X, float* X2, long long nf, int len, long long inc,
+                              float lam, void* stream) {
+    WsGuard guard((cudaStream_t)stream);
+    void* scr = ptvl::lane_scratch(nf, len);
+    if (!scr) return 0;
+    cudaError_t e = ptvl::lane_prox<float>(op, A, B, C, X, nf, len, inc, lam, scr, (cudaStream_t)stream, X2);
+    if (e != cudaSuccess) { cudaGetLastError(); g_err = std::string("proxtv_lane_prox2_dev_f32: ") + cudaGetErrorString(e); return 0; }
+    return 1;
+}
 void proxtv_lane_tuning(int clen, int halo, int variant) { ptvl::lane_set_tuning(clen, halo, variant); }
 void proxtv_lane_tasklog(unsigned long long* dev, long long cap_tasks) { ptvl::lane_set_tasklog(dev, cap_tasks); }
 int proxtv_lane_guard_last(void) { return lane_guard_last(); }

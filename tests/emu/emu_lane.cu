@@ -2,8 +2,8 @@
 // scan steps, window management, sweep, chunk records, verification and repair) on the CPU, one warp task at a time, the 32
 // lanes of a warp in a plain loop (lanes only interact through the warp collectives, which the host Env computes over the
 // loop).  Feed and Drain are the host stand-ins of the kernel's TMA feeder / row drain: same window contents, same calls.
-// Not part of the product; built by tests/test_lane_emulation.py with g++ (host code only; the CUDA headers only supply the
-// __host__ __device__ macros).
+// Not part of the product; built by tests/emu/Makefile with g++ (host code only; the CUDA headers only supply the __host__
+// __device__ macros), from __graft_entry__.build() or on first use by the tests (tests/emu/lane_emu.py).
 #include "../../proxtv_b200/csrc/lane_core.cuh"
 #include <vector>
 #include <string.h>
@@ -204,5 +204,9 @@ void emu_slope_seq_f64(const double* y, int n, double lam, double* x, long long*
     slope_seq<double>(n, lam, 0, LK_BEGIN, [&](int i) { st++; return y[i]; },
                       [&](int f, int e, double v, int) { for (int r = f; r <= e; r++) x[r] = v; return false; });
     if (steps) *steps = st;
+}
+// the same, one fiber after the other over nf fibers stored back to back (the reference of the GPU tests, tests/test_gpu_lane.py)
+void emu_slope_seq_rows_f64(const double* y, long long nf, int n, double lam, double* x) {
+    for (long long j = 0; j < nf; j++) emu_slope_seq_f64(y + j * n, n, lam, x + j * n, nullptr);
 }
 }

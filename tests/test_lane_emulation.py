@@ -10,37 +10,19 @@ repair path takes over), the boxed drain of the contiguous layout, partial fiber
 alternating / integer-valued data, lambda from 0 to 1e4, float32 storage, and the fused Douglas-Rachford pass arithmetic driven
 through a complete DR2_TV solve against the oracle."""
 import ctypes as C
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-EMU_DIR = os.path.join(HERE, "emu")
+from emu import lane_emu
+
 dp = C.POINTER(C.c_double)
 fp = C.POINTER(C.c_float)
 
 
 @pytest.fixture(scope="module")
 def emu():
-    so = os.path.join(EMU_DIR, "libptv_emu_lane.so")
-    src = os.path.join(EMU_DIR, "emu_lane.cu")
-    core = os.path.join(HERE, "..", "proxtv_b200", "csrc", "lane_core.cuh")
-    if not os.path.exists(so) or any(os.path.getmtime(f) > os.path.getmtime(so) for f in (src, core)):
-        cuda_inc = "/usr/local/cuda/include"
-        if not os.path.isdir(cuda_inc):
-            pytest.skip("CUDA headers not available")
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-I" + cuda_inc, "-fPIC", "-ffp-contract=off", "-shared", "-x", "c++", src, "-o", so])
-    lib = C.CDLL(so)
-    lib.emu_lane_f64.argtypes = [C.c_int, dp, dp, dp, dp, dp, C.c_longlong, C.c_int, C.c_longlong, C.c_double, C.c_int, C.c_int, C.c_int, C.c_int,
-                                 C.POINTER(C.c_longlong)]
-    lib.emu_lane_f32.argtypes = [C.c_int, fp, fp, fp, fp, fp, C.c_longlong, C.c_int, C.c_longlong, C.c_float, C.c_int, C.c_int, C.c_int, C.c_int,
-                                 C.POINTER(C.c_longlong)]
-    lib.emu_slope_seq_f64.argtypes = [dp, C.c_int, C.c_double, dp, C.POINTER(C.c_longlong)]
-    lib.emu_plan.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]
-    lib.emu_taskplan.argtypes = [C.c_int, C.c_longlong, C.c_longlong]; lib.emu_taskplan.restype = C.c_longlong
-    return lib
+    return lane_emu.load(required=False)
 
 
 def _p(a, t=dp):
